@@ -48,7 +48,15 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="enqueue the step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU budget of the cpu_baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (its loss and every parameter gradient) as "
+                         "DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -146,6 +154,24 @@ def measured_peaks():
             p = json.load(f)
         return float(p["hbm_gbs"]), float(p.get("bf16_tflops_sustained", p.get("bf16_tflops", 0))), "measured"
     return 6650.0, 1590.0, "fallback"        # B200_PROFILING.md fallback
+
+
+DUMP_BYTES = 60_000_000      # payload of --dump-outputs: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: float32 array} as out_dir/<name>.npy.  When they hold more than DUMP_BYTES, every array is cut to
+    the same fraction of its entries, a fixed sample seeded by its size (flattened, in index order), so that the
+    files of two runs with the same arguments still correspond entry for entry."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    keep = min(1.0, DUMP_BYTES / total) if total else 1.0
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if keep < 1.0:
+            idx = np.random.default_rng(a.size).choice(a.size, int(a.size * keep), replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def pick_engine(requested):
@@ -377,6 +403,12 @@ def run_b200(args):
         step.run()
         ev[k][1].record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        # before the e2e leg below, whose optimizer steps move the parameters
+        names = {id(p): n for n, p in model.named_parameters()}
+        outputs = {"loss": step.loss.cpu().numpy()}
+        outputs.update((f"grad.{names[id(p)]}", g.cpu().numpy()) for p, g in zip(step.params, step.grad_views))
+        dump_outputs(args.dump_outputs, outputs)
     launches = step.launches_per_step * args.steps
     t_ms = sum(a.elapsed_time(b) for a, b in ev)
     t = torch.tensor([t_ms], device=dev, dtype=torch.float64)

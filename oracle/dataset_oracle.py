@@ -2,9 +2,8 @@
 
 SURVEY 8f row n3: `dataset.py` of cmhungsteve/TA3N decides which pre-extracted frame features of a video
 feed the path.  This file restates those rules (plain Python / numpy), each function citing the reference
-lines it follows; `tests/test_dataset.py` pins it against the live reference (when /root/reference is
-present) and against `tests/golden/dataset_indices.npz`, which `oracle/gen_golden_dataset.py` produced by
-running the reference itself.  Only tests may import this module.
+lines it follows; `tests/test_dataset.py` pins it against `tests/golden/dataset_indices.npz`, which
+`oracle/gen_golden_dataset.py` produced by running the reference itself.  Only tests may import this module.
 """
 from __future__ import annotations
 

@@ -11,6 +11,7 @@ import os
 import sys
 
 import numpy as np
+import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
@@ -25,6 +26,23 @@ NEW_LENGTH = [1, 5]
 
 def grid():
     return [(nf, ns, nl) for nl in NEW_LENGTH for ns in SEGMENTS for nf in FRAMES]
+
+
+def make_tree(root, n_videos=7, feat_dim=16, seed=3):
+    """A miniature dataset in the reference's on-disk format: <root>/vK/img_00001.t7 ... one tensor per frame."""
+    g = torch.Generator().manual_seed(seed)
+    lines = []
+    for v in range(n_videos):
+        nf = int(torch.randint(2, 14, (1,), generator=g))
+        d = os.path.join(root, f"v{v}")
+        os.makedirs(d)
+        for f in range(1, nf + 1):
+            torch.save(torch.randn(feat_dim, generator=g), os.path.join(d, "img_{:05d}.t7".format(f)))
+        lines.append(f"{d} {nf} {v % 3}")
+    lst = os.path.join(root, "list.txt")
+    with open(lst, "w") as fh:
+        fh.write("\n".join(lines) + "\n")
+    return lst
 
 
 def reference_dataset(num_segments, new_length, tmp_list):

@@ -16,11 +16,11 @@ plus the loss composition that main.py applies right after it.  Each function
 cites the reference file:line it follows (paths relative to /root/reference).
 
 Parity pinning: the reference ships no tests or golden vectors (SURVEY.md §4),
-so this oracle is pinned against the *live* reference, imported unmodified in
-the build container through ``oracle/ref_shims.py``:
-  * ``tests/test_oracle_vs_reference.py`` compares every output and every
-    parameter gradient of this file with the reference classes (skipped when
-    /root/reference is absent, e.g. on the GPU box);
+so this oracle is pinned against what the reference itself computes, imported
+unmodified through ``oracle/ref_shims.py``:
+  * ``oracle/gen_reference_checks.py`` ran the reference classes to produce
+    ``tests/golden/reference_checks.npz``; ``tests/test_oracle_vs_reference.py``
+    compares every output and every parameter gradient of this file with it;
   * ``oracle/gen_golden.py`` ran the reference to produce ``tests/golden/*.npz``;
     ``tests/test_oracle_golden.py`` checks this oracle against those fixtures
     everywhere.

@@ -7,6 +7,8 @@ import os
 import numpy as np
 import torch
 
+from oracle.gen_reference_checks import pick
+
 GOLDEN_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ta3n_golden.npz")
 
 # Tolerance of the path (north_star): 1e-3 *normwise* relative per tensor, fp32 (SURVEY §8c).
@@ -49,6 +51,46 @@ def assert_close(a, b, tol, what="", noise=0.0):
     assert d <= bound or (den == 0 and d == 0), \
         f"{what}: ||diff||={d:.3e} > {tol:.1e}*||ref||({den:.3e}) + 8*noise({float(noise):.3e})"
     return d / den if den > 0 else d
+
+
+REFERENCE_CHECKS_PATH = os.path.join(os.path.dirname(GOLDEN_PATH), "reference_checks.npz")
+
+
+class ReferenceCheck:
+    """One check of ``reference_checks.npz`` (oracle/gen_reference_checks.py): what the reference computed, by
+    name -- each tensor in full, or a fixed sample of its entries and the norm of the whole tensor."""
+
+    def __init__(self, name: str):
+        z = np.load(REFERENCE_CHECKS_PATH)
+        self.meta = json.loads(bytes(z["meta_json"]).decode())["checks"][name]
+        self.index = self.meta.get("tensors", {})
+        self.values = z[name] if self.index else None
+
+    def names(self, prefix: str):
+        return [k[len(prefix):] for k in self.index if k.startswith(prefix)]
+
+    def norm(self, key: str) -> float:
+        return self.index[key]["norm"]
+
+    def _picked(self, key):
+        e = self.index[key]
+        return self.values[e["offset"]:e["offset"] + e["n"]]
+
+    def __getitem__(self, key) -> torch.Tensor:
+        """The whole tensor (only for tensors stored in full)."""
+        e = self.index[key]
+        assert e["n"] == int(np.prod(e["shape"])), f"{key} is stored as a sample"
+        return torch.from_numpy(self._picked(key).copy()).reshape(e["shape"])
+
+    def assert_close(self, key, got, tol, what=""):
+        """assert_close of the stored entries; for a sampled tensor also ||got|| against the stored norm."""
+        e = self.index[key]
+        assert list(got.shape) == e["shape"], (what, tuple(got.shape), e["shape"])
+        err = assert_close(pick(got), self._picked(key), tol, what)
+        if e["n"] < got.numel():
+            got_norm = got.detach().double().norm().item()
+            assert abs(got_norm - e["norm"]) <= tol * e["norm"], f"{what}: norm {got_norm:.6e} vs {e['norm']:.6e}"
+        return err
 
 
 def sample(t: torch.Tensor, stride: int):

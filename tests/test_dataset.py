@@ -1,5 +1,6 @@
 """Input pipeline (SURVEY 8f n3): segment-index rules, the TSNDataSet drop-in, packed shards and the paired loader.
-CPU only.  Golden index tables come from the unmodified reference (oracle/gen_golden_dataset.py)."""
+CPU only.  Golden index tables and items come from the unmodified reference (oracle/gen_golden_dataset.py,
+oracle/gen_reference_checks.py)."""
 import os
 
 import numpy as np
@@ -8,8 +9,9 @@ import torch
 
 from oracle import dataset_oracle as dorc
 from oracle import gen_golden_dataset as gg
-from oracle import ref_shims
+from oracle import gen_reference_checks as grc
 from ta3n_b200 import dataset as D
+from tests.golden_util import ReferenceCheck
 
 GOLDEN = np.load(gg.GOLDEN_PATH)
 RULES = {"val": (D.val_segment_indices, dorc.val_indices), "test": (D.test_segment_indices, dorc.test_indices),
@@ -34,42 +36,26 @@ def test_index_rules_match_reference_golden(rule):
                 assert got.shape == want.shape and np.array_equal(got.astype(np.int64), want), (rule, key, fn.__module__)
 
 
-def _make_tree(root, n_videos=7, feat_dim=16, seed=3):
-    """A miniature dataset in the reference's on-disk format: <root>/vK/img_00001.t7 ... one tensor per frame."""
-    g = torch.Generator().manual_seed(seed)
-    lines = []
-    for v in range(n_videos):
-        nf = int(torch.randint(2, 14, (1,), generator=g))
-        d = os.path.join(root, f"v{v}")
-        os.makedirs(d)
-        for f in range(1, nf + 1):
-            torch.save(torch.randn(feat_dim, generator=g), os.path.join(d, "img_{:05d}.t7".format(f)))
-        lines.append(f"{d} {nf} {v % 3}")
-    lst = os.path.join(root, "list.txt")
-    with open(lst, "w") as fh:
-        fh.write("\n".join(lines) + "\n")
-    return lst
-
-
-@pytest.mark.skipif(not ref_shims.available(), reason="/root/reference not present")
-@pytest.mark.parametrize("mode", ["test", "val", "random"])
+@pytest.mark.parametrize("mode", grc.TSN_MODES)
 def test_tsn_dataset_equals_live_reference(tmp_path, mode):
-    lst = _make_tree(str(tmp_path))
-    ref_mod = ref_shims.load_dataset()
+    """Item for item, the frames and label the reference's TSNDataSet returned for the same tree and seeds
+    (stored by oracle/gen_reference_checks.py)."""
+    ref = ReferenceCheck(f"tsn/{mode}").meta
+    lst = gg.make_tree(str(tmp_path))
     kw = dict(num_dataload=10, num_segments=5, new_length=1, modality="RGB",
               random_shift=(mode == "random"), test_mode=(mode == "test"))
-    ref, mine = ref_mod.TSNDataSet("", lst, **kw), D.TSNDataSet("", lst, **kw)
-    assert len(ref) == len(mine) == 10                         # list tiled to num_dataload (dataset.py:70-75)
-    for i in range(len(ref)):
-        np.random.seed(100 + i)
-        xr, yr = ref[i]
+    mine = D.TSNDataSet("", lst, **kw)
+    assert ref["len"] == len(mine) == 10                       # list tiled to num_dataload (dataset.py:70-75)
+    for i in range(len(mine)):
         np.random.seed(100 + i)
         xm, ym = mine[i]
-        assert yr == ym and torch.equal(xr, xm), (mode, i)
+        xr = torch.stack([torch.load(os.path.join(str(tmp_path), f"v{v}", "img_{:05d}.t7".format(f)))
+                          for v, f in ref["frames"][i]]).reshape(ref["item_shape"])
+        assert ref["labels"][i] == ym and torch.equal(xr, xm), (mode, i)
 
 
 def test_packed_shard_serves_the_same_items(tmp_path):
-    lst = _make_tree(str(tmp_path))
+    lst = gg.make_tree(str(tmp_path))
     shard = os.path.join(str(tmp_path), "source_T5.npy")
     shape = D.pack_list(lst, shard, num_segments=5)
     assert shape == (7, 5, 16)
@@ -86,7 +72,7 @@ def test_packed_shard_serves_the_same_items(tmp_path):
 
 
 def test_gather_fills_the_staging_buffer_in_batch_order(tmp_path):
-    lst = _make_tree(str(tmp_path))
+    lst = gg.make_tree(str(tmp_path))
     shard = os.path.join(str(tmp_path), "g.npy")
     D.pack_list(lst, shard, num_segments=5)
     packed = D.PackedTSNDataSet(shard, num_dataload=11)
@@ -106,7 +92,7 @@ def test_gather_fills_the_staging_buffer_in_batch_order(tmp_path):
 def test_paired_loader_covers_each_epoch_like_zip_of_random_samplers(tmp_path):
     src_root, tgt_root = os.path.join(str(tmp_path), "s"), os.path.join(str(tmp_path), "t")
     os.makedirs(src_root), os.makedirs(tgt_root)
-    ls, lt = _make_tree(src_root, n_videos=9, seed=1), _make_tree(tgt_root, n_videos=5, seed=2)
+    ls, lt = gg.make_tree(src_root, n_videos=9, seed=1), gg.make_tree(tgt_root, n_videos=5, seed=2)
     D.pack_list(ls, os.path.join(src_root, "p.npy"), 3)
     D.pack_list(lt, os.path.join(tgt_root, "p.npy"), 3)
     # main.py:145-153 tiles the shorter list so that both loaders have the same number of iterations
@@ -132,7 +118,7 @@ def test_paired_loader_covers_each_epoch_like_zip_of_random_samplers(tmp_path):
 
 def test_loader_staging_buffers_are_not_overwritten_early(tmp_path):
     """A yielded batch must stay intact while the next one is consumed (async H2D copies read it)."""
-    lst = _make_tree(str(tmp_path), n_videos=12, seed=7)
+    lst = gg.make_tree(str(tmp_path), n_videos=12, seed=7)
     shard = os.path.join(str(tmp_path), "p.npy")
     D.pack_list(lst, shard, 3)
     ds = D.PackedTSNDataSet(shard)
